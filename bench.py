@@ -33,6 +33,7 @@ import time
 ROOT = os.path.dirname(os.path.abspath(__file__))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True          # the benchmark leaves the tree it runs from as it found it (it may be read-only)
 
 METRIC = "ensemble volumes/sec (inference, fwd+bwd train) at 1/2/4/8 B200 vs CPU ref"
 UNIT = "volumes/s"
@@ -62,7 +63,15 @@ def parse():
     ap.add_argument("--cpu-budget", type=float, default=240.0, help="seconds the --impl reference arm may run")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--graphs", type=int, default=1, help="replay the step from a CUDA graph (vit3d_b200.graphs)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the headline's last timed step returned as DIR/<name>.npy "
+                         "(float32; arrays over their share of 64 MB as a fixed, seeded sample of their elements)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of the GPU path (--impl ours)")
+    return args
 
 
 # ----------------------------------------------------------------------------- clocks
@@ -237,8 +246,9 @@ def time_region(ctx, fn, steps, warm, counter=None):
     return ms, n1 - n0
 
 
-def run_leg(ctx, args, key, steps, warmup, precision, with_u8=True):
-    """Builds one workload, times its device-resident loop and its end-to-end loop.  Returns a dict."""
+def run_leg(ctx, args, key, steps, warmup, precision, with_u8=True, dump_dir=None):
+    """Builds one workload, times its device-resident loop and its end-to-end loop.  Returns a dict.
+    `dump_dir`: write the outputs of the last timed device-resident step there (dump_outputs)."""
     import torch
     import vit3d_b200
     from oracle import vit3d_oracle as O          # test infrastructure: synthetic inputs / seeded weights only
@@ -292,15 +302,20 @@ def run_leg(ctx, args, key, steps, warmup, precision, with_u8=True):
         # train_baseline_cv.py:168-169); every rank holds the same synthetic labels, so local == global
         return batch_pos_weight(y_host)
 
-    def step_dev(x, y):
+    def step_out(x, y):
+        """One step; returns what the caller of the timed path receives."""
         if train:
             return graphed(x, y, pos_weight())
         if sharded is not None:
             return sharded(x)
         if graphed is not None:
-            return graphed(x)[0]
+            return graphed(x)
         with torch.no_grad():
-            return model(x)[0]
+            return model(x)
+
+    def step_dev(x, y):
+        out = step_out(x, y)
+        return out[0] if isinstance(out, tuple) else out
 
     def counter():
         n = L.vit3d_launch_count()
@@ -308,7 +323,23 @@ def run_leg(ctx, args, key, steps, warmup, precision, with_u8=True):
             n += g.replays * g.launches_per_replay
         return n
 
-    ms_dev, launches = time_region(ctx, lambda: step_dev(x_dev, y_dev), steps, warmup, counter)
+    last = [None]
+
+    def timed_step():
+        last[0] = step_out(x_dev, y_dev)
+
+    ms_dev, launches = time_region(ctx, timed_step, steps, warmup, counter)
+    if dump_dir is not None and rank == 0:
+        # before the end-to-end loop below overwrites the graphs' static output buffers
+        if train:
+            arrays = {"loss": last[0], "params": torch.cat([p.detach().reshape(-1) for p in model.parameters()])}
+        elif isinstance(last[0], tuple):        # VisionTransformer.forward: (logits, attention weights, encoded)
+            logits, attn, enc = last[0]
+            arrays = {"logits": logits, **{f"attn_weights_{i}": a for i, a in enumerate(attn)}, "encoded": enc}
+        else:                                   # the ensemble's meta-classifier output
+            arrays = {"out": last[0]}
+        dump_outputs(dump_dir, arrays)
+    del last
 
     # ---- end to end: every step copies ITS batch from pinned host memory (copy stream, double buffered so the copy of
     # step s+1 overlaps the compute of step s), runs the public call and reads the result back before it counts as done
@@ -401,6 +432,26 @@ def run_leg(ctx, args, key, steps, warmup, precision, with_u8=True):
     del model, members, graphed, sharded, opt
     torch.cuda.empty_cache()
     return out
+
+
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(path, arrays):
+    """Writes every tensor of `arrays` (name -> tensor) as `path`/<name>.npy in float32, DUMP_BYTES in all.  A tensor
+    larger than its share is written as the flat sample of its elements at sorted indices drawn from a generator
+    seeded with 0: the same indices for the same shapes, so two builds run with the same arguments compare element
+    for element."""
+    import numpy as np
+    import torch
+    os.makedirs(path, exist_ok=True)
+    cap = DUMP_BYTES // 4 // len(arrays)
+    for name, t in arrays.items():
+        t = t.detach().float()
+        if t.numel() > cap:
+            idx = torch.randint(t.numel(), (cap,), generator=torch.Generator().manual_seed(0)).unique()
+            t = t.reshape(-1)[idx.to(t.device)]
+        np.save(os.path.join(path, name + ".npy"), t.cpu().numpy())
 
 
 def ensemble_small_batch_probe(ctx, args):
@@ -537,7 +588,7 @@ def main():
     clocks = ClockSampler(local_rank)
     if rank == 0:
         clocks.start()
-    head = run_leg(ctx, args, args.workload, args.steps, args.warmup, args.precision)
+    head = run_leg(ctx, args, args.workload, args.steps, args.warmup, args.precision, dump_dir=args.dump_outputs)
     clk = clocks.stop() if rank == 0 else None
     head_ctx = ctx.last
 

@@ -4,13 +4,12 @@ import ctypes
 import os
 import re
 
-import numpy as np
 import pytest
 import torch
 
 import vit3d_b200
 from oracle import vit3d_oracle as O
-from tests.helpers import CASES, load_golden, stats
+from tests.helpers import CASES, assert_stats_equal, load_golden, stats
 from vit3d_b200 import _lib
 from vit3d_b200.models.modeling import (Attention, Block, Embeddings, Encoder, Mlp, Transformer, TransformerEnsemble,
                                         VisionTransformer)
@@ -30,7 +29,7 @@ def test_constructor_matches_reference_rng_and_keys(name):
     keys = sorted(k[len(name) + 1:] for k in g.files if k.startswith(name + "/"))
     assert sorted(sd.keys()) == keys
     for k in keys:
-        np.testing.assert_array_equal(stats(sd[k]), g[f"{name}/{k}"], err_msg=k)
+        assert_stats_equal(stats(sd[k]), g[f"{name}/{k}"], k)
 
 
 def test_state_dict_roundtrip_with_oracle_layout():
@@ -96,7 +95,7 @@ def test_product_does_not_import_oracle():
                 assert "vit3d_oracle" not in src, f
 
 
-def test_reference_import_line_works_with_package_dir_on_sys_path():
+def test_reference_import_line_works_with_package_dir_on_sys_path(tmp_path):
     """`from models.modeling import VisionTransformer` (train_baseline_cv.py:14) resolves to this
     implementation when 3d_vit_ensemble_b200/ is on sys.path, with the SAME class objects."""
     import subprocess
@@ -105,5 +104,5 @@ def test_reference_import_line_works_with_package_dir_on_sys_path():
             "from models.modeling import VisionTransformer, TransformerEnsemble; "
             "import importlib; v = importlib.import_module('3d_vit_ensemble_b200.vit'); "
             "assert VisionTransformer is v.VisionTransformer; print('ok')") % os.path.join(ROOT, "3d_vit_ensemble_b200")
-    r = subprocess.run([sys.executable, "-c", code], capture_output=True, text=True, cwd="/tmp")
+    r = subprocess.run([sys.executable, "-c", code], capture_output=True, text=True, cwd=tmp_path)
     assert r.returncode == 0 and "ok" in r.stdout, r.stderr

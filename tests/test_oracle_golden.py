@@ -7,7 +7,7 @@ import pytest
 import torch
 
 from oracle import vit3d_oracle as O
-from tests.helpers import CASES, assert_stats_close, case_setup, load_golden, stats, unpack_masks
+from tests.helpers import CASES, assert_stats_close, assert_stats_equal, case_setup, load_golden, stats, unpack_masks
 
 FAST = ["tiny", "shipped", "conf5", "conf18", "shipped_p8"]
 
@@ -20,16 +20,16 @@ def test_init_matches_reference_constructor_rng():
         keys = [k[len(name) + 1:] for k in g.files if k.startswith(name + "/")]
         assert sorted(keys) == sorted(sd.keys())
         for k in keys:
-            np.testing.assert_allclose(stats(sd[k]), g[f"{name}/{k}"], rtol=0, atol=0, err_msg=f"{name}/{k}")
+            assert_stats_equal(stats(sd[k]), g[f"{name}/{k}"], f"{name}/{k}")
 
 
 @pytest.mark.parametrize("name", list(CASES))
 def test_forward_matches_reference(name):
     g = load_golden(name)
     cfg, sd, x, y, w = case_setup(name)
-    np.testing.assert_array_equal(stats(x), g["x_stats"])
+    assert_stats_equal(stats(x), g["x_stats"], "x")
     for k, v in sd.items():
-        np.testing.assert_array_equal(stats(v), g["sd_stats/" + k], err_msg=k)
+        assert_stats_equal(stats(v), g["sd_stats/" + k], k)
     logits, probs, enc = O.vit_forward(sd, cfg, x)
     np.testing.assert_allclose(logits.numpy(), g["logits"], atol=2e-5, rtol=0)
     np.testing.assert_allclose(enc[:, 0].numpy(), g["cls_feature"], atol=5e-5, rtol=0)

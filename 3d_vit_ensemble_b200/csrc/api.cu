@@ -1,9 +1,6 @@
 // extern "C" surface of libvit3d_sm100.so (declared in include/vit3d.h): argument checks and
 // dispatch between the tcgen05 kernels and the shape-generic fp32 kernels.
 #include <stdarg.h>
-#include <stdlib.h>
-
-#include <mutex>
 
 #include "common.cuh"
 #include "kernels.cuh"
@@ -38,33 +35,31 @@ int sm_count() {
   return cached;
 }
 
-// tuning switches: A/B selection of kernel variants without rebuilding (defaults: environment, else built-in)
-// (process-wide; read and written with relaxed atomics, initialised exactly once: the entry points are re-entrant)
-static int g_tuning[VIT3D_TUNE_COUNT];
-static std::once_flag g_tuning_once;
-static void tuning_defaults() {
-  std::call_once(g_tuning_once, [] {
-    auto env = [](const char* name, int dflt) { const char* e = getenv(name); return e ? atoi(e) : dflt; };
-    auto set = [](int key, int v) { __atomic_store_n(&g_tuning[key], v, __ATOMIC_RELAXED); };
-    set(VIT3D_TUNE_EPI_PANEL, env("VIT3D_EPI_PANEL", 1));
-    set(VIT3D_TUNE_EPI_LEAN, env("VIT3D_EPI_LEAN", 1));
-    set(VIT3D_TUNE_STORE_WIDE, env("VIT3D_STORE_WIDE", 0));
-    set(VIT3D_TUNE_L2_AHEAD, env("VIT3D_L2_AHEAD", 0));
-    set(VIT3D_TUNE_MLP_PAIR, env("VIT3D_MLP_PAIR", 0));
-    set(VIT3D_TUNE_WGRAD_RED, env("VIT3D_WGRAD_RED", 1));
-    set(VIT3D_TUNE_ATTN_BWD, env("VIT3D_ATTN_BWD", 1));
-    set(VIT3D_TUNE_RES_PAIR, env("VIT3D_RES_PAIR", 0));
-    set(VIT3D_TUNE_ATTN_TF32, env("VIT3D_ATTN_TF32", 1));
-    set(VIT3D_TUNE_F32_BOX, env("VIT3D_F32_BOX", 0));
-    set(VIT3D_TUNE_PATCH_TALL, env("VIT3D_PATCH_TALL", 0));
-    set(VIT3D_TUNE_PATCH_CLUSTER, env("VIT3D_PATCH_CLUSTER", 0));
-    set(VIT3D_TUNE_PATCH_TF32, env("VIT3D_PATCH_TF32", 1));
-    set(VIT3D_TUNE_ATTN_FWD_UNIT, env("VIT3D_ATTN_FWD_UNIT", 0));
-    set(VIT3D_TUNE_ATTN_THREADS, env("VIT3D_ATTN_THREADS", 0));
-  });
-}
+// tuning switches (test and probe hooks, include/vit3d.h), indexed by key; process-wide, read and written with
+// relaxed atomics (the entry points are re-entrant).  Retired keys keep their slot but can be neither set nor read.
+static int g_tuning[VIT3D_TUNE_COUNT] = {
+    0,  //  0 retired
+    0,  //  1 ATTN_THREADS
+    0,  //  2 retired
+    0,  //  3 retired
+    0,  //  4 retired
+    0,  //  5 MLP_PAIR
+    1,  //  6 WGRAD_RED
+    1,  //  7 ATTN_BWD
+    0,  //  8 RES_PAIR
+    1,  //  9 ATTN_TF32
+    0,  // 10 retired
+    0,  // 11 PATCH_TALL
+    0,  // 12 PATCH_CLUSTER
+    0,  // 13 retired
+    0,  // 14 ATTN_FWD_UNIT
+};
+constexpr unsigned kLiveTuningKeys =
+    1u << VIT3D_TUNE_ATTN_THREADS | 1u << VIT3D_TUNE_MLP_PAIR | 1u << VIT3D_TUNE_WGRAD_RED | 1u << VIT3D_TUNE_ATTN_BWD |
+    1u << VIT3D_TUNE_RES_PAIR | 1u << VIT3D_TUNE_ATTN_TF32 | 1u << VIT3D_TUNE_PATCH_TALL | 1u << VIT3D_TUNE_PATCH_CLUSTER |
+    1u << VIT3D_TUNE_ATTN_FWD_UNIT;
+static bool tuning_key_live(int key) { return key >= 0 && key < VIT3D_TUNE_COUNT && ((kLiveTuningKeys >> key) & 1u); }
 int tuning(int key) {
-  tuning_defaults();
   return (key >= 0 && key < VIT3D_TUNE_COUNT) ? __atomic_load_n(&g_tuning[key], __ATOMIC_RELAXED) : 0;
 }
 
@@ -89,12 +84,14 @@ int vit3d_device_info(int* sms, int* cc) {
   return VIT3D_OK;
 }
 int vit3d_set_tuning(int key, int value) {
-  V3_REQUIRE(key >= 0 && key < VIT3D_TUNE_COUNT, "set_tuning: unknown key %d", key);
-  tuning_defaults();
+  V3_REQUIRE(tuning_key_live(key), "set_tuning: unknown or retired key %d", key);
   __atomic_store_n(&g_tuning[key], value, __ATOMIC_RELAXED);
   return VIT3D_OK;
 }
-int vit3d_get_tuning(int key) { return tuning(key); }
+int vit3d_get_tuning(int key) {
+  V3_REQUIRE(tuning_key_live(key), "get_tuning: unknown or retired key %d", key);
+  return tuning(key);
+}
 unsigned long long vit3d_launch_count(void) { return __atomic_load_n(&g_launches, __ATOMIC_RELAXED); }
 int vit3d_act_bytes(int prec) { return prec == VIT3D_PREC_BF16 ? 2 : 4; }
 int vit3d_tc_supported(int prec, int M, int N, int K) { return tc_linear_supported(prec, M, N, K) ? 1 : 0; }
@@ -133,7 +130,7 @@ int vit3d_patch_embed_fwd(const float* x, const float* w, const float* bias, con
     return launch_cls_rows(cls, pos, tokens, B, S, H, st);
   }
   V3_REQUIRE(ws && ws_bytes >= vit3d_patch_embed_ws_bytes(B, X, Y, Z, p0, p1, p2, H, prec), "patch_embed_fwd: workspace too small");
-  if (prec == VIT3D_PREC_TF32 && tuning(VIT3D_TUNE_PATCH_TF32) != 0 && tc_patch_embed_supported(B, X, Y, Z, p0, p1, p2, H) &&
+  if (prec == VIT3D_PREC_TF32 && tc_patch_embed_supported(B, X, Y, Z, p0, p1, p2, H) &&
       (size_t)B * X * Y * Z * sizeof(float) <= ws_bytes) {
     // TF32 mode: the volume is rounded to nearest TF32 into the workspace first (the tensor core would truncate the raw
     // input), then takes the same TMA-im2col tensor-core GEMM as BF16 mode: every GEMM operand of this mode is an

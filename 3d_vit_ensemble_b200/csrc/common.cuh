@@ -46,7 +46,7 @@ void count_launch();
 static inline cudaStream_t as_stream(vit3d_stream_t s) { return reinterpret_cast<cudaStream_t>(s); }
 static inline int ceil_div(long long a, long long b) { return (int)((a + b - 1) / b); }
 int sm_count();
-// run-time tuning switches (vit3d_set_tuning; defaults from the environment, see include/vit3d.h)
+// run-time tuning switches (test and probe hooks set by vit3d_set_tuning, see include/vit3d.h)
 int tuning(int key);
 
 // ----------------------------------------------------------------------------- programmatic dependent launch

@@ -44,10 +44,12 @@ template <int BN> struct TcCfg {
   static constexpr int TMEM_COLS = 2 * BN;
   static constexpr int EPI_WARPS = tc_epi_warps(BN);
   static constexpr int THREADS = tc_threads(BN);
-  static constexpr int EPI_BYTES = EPI_WARPS * 2048;   // one 32-row x 64-byte transpose tile per epilogue warp
+  static constexpr int EPI_WARP_BYTES = 2048;          // one 32-row x 64-byte transpose tile per epilogue warp
+  static constexpr int EPI_BYTES = EPI_WARPS * EPI_WARP_BYTES;
   static constexpr int BIAS_BYTES = BN * 6;            // the n-tile's bias: fp32 copy + packed-half copy
   static constexpr int SMEM_BYTES = OPER_BYTES + EPI_BYTES + BIAS_BYTES + 256 /*barriers*/;
   static_assert(OPER_BYTES >= TC_SLAB_BYTES + TC_STAT_STAGES * A_BYTES, "operand region too small for the stationary schedule");
+  static_assert(SMEM_BYTES <= 232448, "over the 227 KB shared-memory limit");
 };
 
 // work-item sequence of a CTA (identical in the producer, MMA and epilogue roles)
@@ -99,34 +101,19 @@ struct TileIter {
 
 // EPI: EPI_GENERIC (run-time epilogue flags) or the compile-time mode of epilogue_bf16_lean.
 // 18 warps = 5 on one scheduler: 16384 / (5 * 32) -> at most 96 registers per thread (ptxas derives this).
-// WIDE (lean bf16 epilogue, BN = 256): 4 KB staging panel per epilogue warp (128-byte output rows); the
-// operand region shrinks to slab + 2 A stages (stationary) or 3 stages (streaming) to make room.
-template <int BN, bool WIDE> struct TcLayout {
-  using Cfg = TcCfg<BN>;
-  static constexpr int STAT_STAGES = WIDE ? 2 : TC_STAT_STAGES;
-  static constexpr int STREAM_STAGES = WIDE ? 3 : Cfg::STAGES;
-  static constexpr int OPER_BYTES = WIDE ? TC_SLAB_BYTES + 2 * Cfg::A_BYTES : Cfg::OPER_BYTES;
-  static constexpr int EPI_WARP_BYTES = WIDE ? 4096 : 2048;
-  static constexpr int EPI_BYTES = Cfg::EPI_WARPS * EPI_WARP_BYTES;
-  static constexpr int SMEM_BYTES = OPER_BYTES + EPI_BYTES + Cfg::BIAS_BYTES + 256 /*barriers*/;
-  static_assert(!WIDE || STREAM_STAGES * Cfg::STAGE_BYTES <= OPER_BYTES, "streaming ring does not fit");
-  static_assert(SMEM_BYTES <= 232448, "over the 227 KB shared-memory limit");
-};
-
-template <bool TF32, int BN, int EPI = EPI_GENERIC, bool WIDE = false>
+template <bool TF32, int BN, int EPI = EPI_GENERIC>
 __global__ void __launch_bounds__(tc_threads(BN), 1)
 tc_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmB,
                const __grid_constant__ CUtensorMap tmC, const __grid_constant__ CUtensorMap tmPre,
                const __grid_constant__ CUtensorMap tmX, TcEpilogue ep, int M, int N, int K, int tiles_m, int tiles_n,
                int splits, int stationary, int patch_blocks, int mn_major) {
   using Cfg = TcCfg<BN>;
-  using Lay = TcLayout<BN, WIDE>;
   constexpr int BLOCK_K = TF32 ? 32 : 64;   // 128 bytes of K per stage row
   extern __shared__ __align__(1024) uint8_t smem_raw[];
   uint8_t* smem = smem_raw;                    // 128B-swizzled operand tiles need 1024-byte alignment
   if (smem_u32(smem) & 1023u) __trap();
-  uint8_t* epi_stage = smem + Lay::OPER_BYTES;
-  uint8_t* bias_stage = epi_stage + Lay::EPI_BYTES;
+  uint8_t* epi_stage = smem + Cfg::OPER_BYTES;
+  uint8_t* bias_stage = epi_stage + Cfg::EPI_BYTES;
   uint64_t* bars = reinterpret_cast<uint64_t*>(bias_stage + Cfg::BIAS_BYTES);
   constexpr int MAXST = 8;
   uint64_t* full_bar = bars;                 // [MAXST]
@@ -139,7 +126,7 @@ tc_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
   const bool stat = stationary != 0;
   const bool tall = (mn_major & 2) != 0;   // 256 x BN tile: the A stage doubles, both TMEM buffers form ONE accumulator pair
   const bool mnm = (mn_major & 1) != 0;    // both operands MN-major (weight gradients)
-  const int STAGES = stat ? Lay::STAT_STAGES : (tall ? Lay::OPER_BYTES / (Cfg::STAGE_BYTES + Cfg::A_BYTES) : Lay::STREAM_STAGES);
+  const int STAGES = stat ? TC_STAT_STAGES : (tall ? Cfg::OPER_BYTES / (Cfg::STAGE_BYTES + Cfg::A_BYTES) : Cfg::STAGES);
   const int stage_bytes = stat ? Cfg::A_BYTES : (tall ? Cfg::STAGE_BYTES + Cfg::A_BYTES : Cfg::STAGE_BYTES);
   uint8_t* ring = stat ? smem + TC_SLAB_BYTES : smem;
 
@@ -184,8 +171,6 @@ tc_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
       }
       int stage = 0;
       uint32_t phase = 0;
-      // L2 look-ahead (tiles): deep-K tiles last long, one tile ahead is enough; K = 256 tiles need ~4
-      const int l2_ahead = (patch_blocks > 0 || mn_major || splits > 1) ? 0 : (nkb <= 8 ? ep.l2_ahead : min(ep.l2_ahead, 1));
       const int a_bytes = tall ? 2 * Cfg::A_BYTES : Cfg::A_BYTES;
       while (ti.next()) {
         const int kb0 = ti.split * kb_per, kb1 = min(nkb, kb0 + kb_per);
@@ -223,11 +208,6 @@ tc_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
           } else {
             tma_load_2d(sa, &tmA, &full_bar[stage], kb * BLOCK_K, ti.tm * TC_BLOCK_M);
             if (!stat) tma_load_2d(sa + Cfg::A_BYTES, &tmB, &full_bar[stage], kb * BLOCK_K, ti.tn * BN);
-            // pull the same k-block of the A tile this CTA will need `l2_ahead` tiles from now into L2
-            if (l2_ahead > 0) {
-              const int tm_ahead = stat ? ti.tm + l2_ahead * ti.cpn : (ti.w + l2_ahead * (int)gridDim.x) / (splits * tiles_n);
-              if (tm_ahead < tiles_m) tma_prefetch_2d(&tmA, kb * BLOCK_K, tm_ahead * TC_BLOCK_M);
-            }
           }
           if (++stage == STAGES) { stage = 0; phase ^= 1; }
         }
@@ -288,7 +268,7 @@ tc_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
     const int q = warp & 3;                 // TMEM lane quarter this warp may read
     const int part = (warp - 2) >> 2;       // which slice of the tile's columns
     constexpr int CW = BN / (Cfg::EPI_WARPS / 4);
-    const uint32_t stage = smem_u32(epi_stage + (warp - 2) * Lay::EPI_WARP_BYTES);
+    const uint32_t stage = smem_u32(epi_stage + (warp - 2) * Cfg::EPI_WARP_BYTES);
     TileIter ti(stat, tiles_m, tiles_n, splits);
     int it = 0;
     int cur_tn = -1;
@@ -340,7 +320,7 @@ tc_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
         mbar_wait(&tmem_full[buf], (it >> 1) & 1);
         tc_fence_after();
         const uint32_t taddr = tmem_base + ((uint32_t)(q * 32) << 16) + buf * BN + part * CW;
-        epilogue_bf16_lean<CW, EPI, WIDE>(&tmC, &tmPre, taddr, stage, smem_u32(bias_stage) + part * CW * 4,
+        epilogue_bf16_lean<CW, EPI>(&tmC, &tmPre, taddr, stage, smem_u32(bias_stage) + part * CW * 4,
                                     smem_u32(bias_stage) + BN * 4 + part * CW * 2, lane, m_base, n_base, keep,
                                     ep.drop_scale);
       } else {
@@ -438,18 +418,17 @@ int make_tmap_2d(CUtensorMap* out, const void* ptr, int elem_bytes, long long ro
   return VIT3D_OK;
 }
 
-template <bool TF32, int BN, int EPI = EPI_GENERIC, bool WIDE = false>
+template <bool TF32, int BN, int EPI = EPI_GENERIC>
 static int launch_tc(const CUtensorMap& ta, const CUtensorMap& tb, const CUtensorMap& tc, const CUtensorMap& tp,
                      const TcEpilogue& ep, int M, int N, int K, int splits, bool stationary, cudaStream_t st,
                      int patch_blocks = 0, int mn_major = 0, const CUtensorMap* tx = nullptr) {
   using Cfg = TcCfg<BN>;
-  using Lay = TcLayout<BN, WIDE>;
-  auto kern = tc_gemm_kernel<TF32, BN, EPI, WIDE>;
+  auto kern = tc_gemm_kernel<TF32, BN, EPI>;
   static thread_local int configured_dev = -1;
   int dev = 0;
   V3_CUDA(cudaGetDevice(&dev));
   if (configured_dev != dev) {
-    V3_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, Lay::SMEM_BYTES));
+    V3_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, Cfg::SMEM_BYTES));
     configured_dev = dev;
   }
   const int tiles_m = ceil_div(M, (mn_major & 2) ? 2 * TC_BLOCK_M : TC_BLOCK_M), tiles_n = ceil_div(N, BN);
@@ -468,22 +447,20 @@ static int launch_tc(const CUtensorMap& ta, const CUtensorMap& tb, const CUtenso
       set_error("tc_gemm: cluster multicast needs grid and tail tile counts that are multiples of the cluster size");
       return VIT3D_ERR_INVALID;
     }
-    V3_CUDA(launch_pdl_cluster(kern, dim3(grid), dim3(Cfg::THREADS), (size_t)Lay::SMEM_BYTES, st, ep.cluster, ta, tb, tc, tp,
+    V3_CUDA(launch_pdl_cluster(kern, dim3(grid), dim3(Cfg::THREADS), (size_t)Cfg::SMEM_BYTES, st, ep.cluster, ta, tb, tc, tp,
                                tx ? *tx : tp, ep, M, N, K, tiles_m, tiles_n, splits, stationary ? 1 : 0, patch_blocks, mn_major));
     V3_LAUNCH_CHECK();
     return VIT3D_OK;
   }
-  V3_CUDA(launch_pdl(kern, dim3(grid), dim3(Cfg::THREADS), (size_t)Lay::SMEM_BYTES, st, ta, tb, tc, tp, tx ? *tx : tp, ep, M, N, K, tiles_m,
+  V3_CUDA(launch_pdl(kern, dim3(grid), dim3(Cfg::THREADS), (size_t)Cfg::SMEM_BYTES, st, ta, tb, tc, tp, tx ? *tx : tp, ep, M, N, K, tiles_m,
                      tiles_n, splits, stationary ? 1 : 0, patch_blocks, mn_major));
   V3_LAUNCH_CHECK();
   return VIT3D_OK;
 }
 
 // D[M,N] = A[M,K] B[N,K]^T with both operands dense row-major K-major; elem = 2 (bf16) or 4 (tf32)
-int tc_gemm(bool tf32, const void* A, const void* B, int M, int N, int K, const TcEpilogue& ep_in, int splits,
+int tc_gemm(bool tf32, const void* A, const void* B, int M, int N, int K, const TcEpilogue& ep, int splits,
             cudaStream_t st) {
-  TcEpilogue ep = ep_in;
-  ep.l2_ahead = tuning(VIT3D_TUNE_L2_AHEAD);
   const int eb = tf32 ? 4 : 2;
   const int sms = sm_count();
   const int tm = ceil_div(M, TC_BLOCK_M);
@@ -503,14 +480,6 @@ int tc_gemm(bool tf32, const void* A, const void* B, int M, int N, int K, const 
   if (rc != VIT3D_OK) return rc;
   tc = ta;
   tp = ta;
-  if (ep.out_f32 && !ep.atomic && ep.row_group == 0 && ep.seg_rows == 0 && !ep.partial_ws && N % 4 == 0 &&
-      (reinterpret_cast<uintptr_t>(ep.out) & 15) == 0 && tuning(VIT3D_TUNE_F32_BOX) != 0) {
-    // fp32 outputs (TF32 mode, fp32 data gradients): [32 x 16] boxes through the TMA unit instead of 64-byte row
-    // segments from the epilogue warps' load/store path
-    rc = make_tmap_2d(&tc, ep.out, 4, M, N, N, 32, 16, 64);
-    if (rc != VIT3D_OK) return rc;
-    ep.f32_box = 1;
-  }
   if (!ep.out_f32) {   // bf16 outputs leave through bulk tensor stores
     if (ep.row_group > 0 || ep.atomic) { set_error("tc_gemm: bf16 output with row remap / atomics is not supported"); return VIT3D_ERR_INVALID; }
     rc = make_tmap_2d(&tc, ep.out, 2, M, N, N, 32, 32, 64);
@@ -526,19 +495,10 @@ int tc_gemm(bool tf32, const void* A, const void* B, int M, int N, int K, const 
     return launch_tc<true, 64>(ta, tb, tc, tp, ep, M, N, K, splits, stationary, st);
   }
   // compile-time specialised epilogue for the hot bf16-output products (full column tiles)
-  if (!ep.out_f32 && bn >= 128 && N % bn == 0 && tuning(VIT3D_TUNE_EPI_LEAN) != 0 &&
+  if (!ep.out_f32 && bn >= 128 && N % bn == 0 &&
       (!ep.pre || ep.act == VIT3D_ACT_GELU) && (ep.act == VIT3D_ACT_NONE || ep.bias) &&
       (!ep.drop_bits || ep.store_dact) && (!ep.store_dact || (ep.pre && ep.bias && ep.act == VIT3D_ACT_GELU))) {
     const int mode = (ep.bias ? 1 : 0) | (ep.act == VIT3D_ACT_GELU ? 2 : 0) | (ep.pre ? 4 : 0) | (ep.store_dact ? 8 : 0);
-    if (bn == 256 && !ep.pre && tuning(VIT3D_TUNE_STORE_WIDE) != 0) {
-      // one [32 x 64] panel (128-byte rows) per epilogue warp and tile
-      CUtensorMap tw;
-      rc = make_tmap_2d(&tw, ep.out, 2, M, N, N, 32, 64, 128);
-      if (rc != VIT3D_OK) return rc;
-      if (mode == 0) return launch_tc<false, 256, 0, true>(ta, tb, tw, tw, ep, M, N, K, splits, stationary, st);
-      if (mode == 1) return launch_tc<false, 256, 1, true>(ta, tb, tw, tw, ep, M, N, K, splits, stationary, st);
-      if (mode == 3) return launch_tc<false, 256, 3, true>(ta, tb, tw, tw, ep, M, N, K, splits, stationary, st);
-    }
 #define V3_LEAN(BN_, MODE_) \
   if (bn == BN_ && mode == MODE_) return launch_tc<false, BN_, MODE_>(ta, tb, tc, tp, ep, M, N, K, splits, stationary, st);
     V3_LEAN(256, 0) V3_LEAN(256, 1) V3_LEAN(256, 3) V3_LEAN(256, 7) V3_LEAN(256, 15)
@@ -686,7 +646,7 @@ int tc_linear_fwd(const TcLinear& t, cudaStream_t st) {
   const bool aligned = ((reinterpret_cast<uintptr_t>(t.y) | reinterpret_cast<uintptr_t>(t.residual) |
                          reinterpret_cast<uintptr_t>(t.ln_out)) & 15) == 0;
   if (t.prec == VIT3D_PREC_BF16 && t.y_f32 && t.act == VIT3D_ACT_NONE && !t.pre && aligned &&
-      tc_res_supported(t.M, t.N, t.K, t.ln_out != nullptr) && (t.ln_out || tuning(VIT3D_TUNE_EPI_PANEL) != 0))
+      tc_res_supported(t.M, t.N, t.K, t.ln_out != nullptr))
     return tc_gemm_res(t, st);
   if (t.ln_out) V3_UNSUPPORTED("linear + LayerNorm: unsupported shape / alignment (M=%d N=%d K=%d)", t.M, t.N, t.K);
   TcEpilogue ep;
@@ -762,7 +722,7 @@ int tc_patch_embed_fwd(const float* x, const float* w, const float* bias, const 
   }
   TcEpilogue ep;
   ep.bias = bias; ep.rowadd = pos; ep.row_group = P; ep.out = tokens; ep.out_f32 = 1; ep.vols_per_tile = vpt;
-  // Optional (VIT3D_PATCH_CLUSTER, off): the filter bank (1.3 MB, re-streamed for every row tile: 32 KB per k-block
+  // Optional (VIT3D_TUNE_PATCH_CLUSTER, off): the filter bank (1.3 MB, re-streamed for every row tile: 32 KB per k-block
   // beside 16 KB of volume data) fetched ONCE per cluster - each CTA loads 1/cl of the filters and multicasts them.
   // The cluster's CTAs share ring slots, so they must walk equally many tiles: the grid is cut to whole co-resident
   // clusters whose tail (total % grid) is a multiple of the cluster size (B200: 74 pairs, but only 33 clusters of 4).
@@ -773,13 +733,13 @@ int tc_patch_embed_fwd(const float* x, const float* w, const float* bias, const 
     for (int cl = tuning(VIT3D_TUNE_PATCH_CLUSTER) >= 4 ? 4 : 2; cl >= 2 && ep.cluster == 1; cl -= 2) {
       int nmax = 0;
       {
-        using Lay = TcLayout<256, false>;
-        auto kern = tc_gemm_kernel<true, 256, EPI_GENERIC, false>;
-        cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, Lay::SMEM_BYTES);
+        using Cfg = TcCfg<256>;
+        auto kern = tc_gemm_kernel<true, 256, EPI_GENERIC>;
+        cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, Cfg::SMEM_BYTES);
         cudaLaunchConfig_t cfg = {};
         cfg.gridDim = dim3(sms - sms % cl);
-        cfg.blockDim = dim3(TcCfg<256>::THREADS);
-        cfg.dynamicSmemBytes = Lay::SMEM_BYTES;
+        cfg.blockDim = dim3(Cfg::THREADS);
+        cfg.dynamicSmemBytes = Cfg::SMEM_BYTES;
         cudaLaunchAttribute attr[1];
         attr[0].id = cudaLaunchAttributeClusterDimension;
         attr[0].val.clusterDim.x = cl; attr[0].val.clusterDim.y = 1; attr[0].val.clusterDim.z = 1;

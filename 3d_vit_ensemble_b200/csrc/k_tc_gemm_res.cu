@@ -44,7 +44,6 @@ struct ResEpilogue {
   float* mean = nullptr;           // [M] optional (LN)
   float* rstd = nullptr;           // [M] optional (LN)
   float eps = 1e-6f;
-  int l2_ahead = 0;                // tiles of A prefetched into L2 ahead of the operand ring
   const uint32_t* drop_bits = nullptr;   // keep bits over [M,N] (MODE bit 3): (A B^T + bias) * keep * drop_scale + residual
   float drop_scale = 1.f;
 };
@@ -120,11 +119,6 @@ tc_gemm_res_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constan
                               tn * RS_BN + (int)rank * (RS_BN / CL), (uint16_t)((1u << CL) - 1u));
           else
             tma_load_2d(sa + RS_A_BYTES, &tmB, &full_bar[stage], kb * 64, tn * RS_BN);
-          // the same k-block of the A tile this CTA handles `l2_ahead` tiles from now -> L2
-          if (ep.l2_ahead > 0) {
-            const int wa = w + (nkb <= 8 ? ep.l2_ahead : 1) * (int)gridDim.x;
-            if (wa < total) tma_prefetch_2d(&tmA, kb * 64, (wa / tiles_n) * RS_BM);
-          }
           if (++stage == RS_STAGES) { stage = 0; phase ^= 1; }
         }
       }
@@ -399,7 +393,6 @@ int tc_gemm_res(const TcLinear& t, cudaStream_t st) {
     if (rc != VIT3D_OK) return rc;
   }
   ResEpilogue ep;
-  ep.l2_ahead = tuning(VIT3D_TUNE_L2_AHEAD);
   ep.bias = t.bias; ep.gamma = t.ln_gamma; ep.beta = t.ln_beta; ep.mean = t.ln_mean; ep.rstd = t.ln_rstd; ep.eps = t.ln_eps;
   ep.drop_bits = t.drop_bits; ep.drop_scale = t.drop_scale;
   const int mode = (t.bias ? 1 : 0) | (t.residual ? 2 : 0) | (ln ? 4 : 0);

@@ -114,14 +114,6 @@ __device__ __forceinline__ void tma_load_2d(void* smem_dst, const CUtensorMap* m
       "l"(reinterpret_cast<uint64_t>(m)), "r"(smem_u32(bar)), "r"(c0), "r"(c1)
       : "memory");
 }
-// L2 prefetch of a tensor box (no shared-memory destination, no completion signal): issued a few tiles ahead
-// of the real load so that the load finds its operand in L2.  Under the write-heavy traffic of these GEMMs a
-// first-touch HBM read takes ~2.5 us, which a 64 KB shared-memory ring cannot cover.
-__device__ __forceinline__ void tma_prefetch_2d(const CUtensorMap* m, int c0, int c1) {
-  asm volatile("cp.async.bulk.prefetch.tensor.2d.L2.global.tile [%0, {%1, %2}];" ::"l"(reinterpret_cast<uint64_t>(m)),
-               "r"(c0), "r"(c1)
-               : "memory");
-}
 __device__ __forceinline__ void tma_load_3d(void* smem_dst, const CUtensorMap* m, uint64_t* bar, int c0, int c1, int c2) {
   asm volatile(
       "cp.async.bulk.tensor.3d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5}], [%2];" ::"r"(

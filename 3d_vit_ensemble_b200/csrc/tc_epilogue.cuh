@@ -22,11 +22,9 @@ struct TcEpilogue {
   int row_group = 0;                // >0: out row = m + m / row_group + 1
   int cluster = 1;                  // patch mode: CTAs of a cluster share every filter-bank k-block by TMA multicast
   int grid_limit = 0;               // > 0: launch at most this many CTAs (cluster launches: whole co-resident clusters)
-  int f32_box = 0;                  // fp32 output leaves as [32 x 16] TMA boxes through tmC (dense rows, no row remap / atomics)
   int atomic = 0;                   // accumulate (split-K): 1 = fp32 vector atomics, 2 = TMA reduce-add boxes (tmC / tmPre / tmX per segment)
   int vols_per_tile = 0;            // patch-embedding mode: volumes per 128-row tile
   int round_tf32 = 0;               // fp32 output is the operand of a TF32 GEMM: round to nearest tf32
-  int l2_ahead = 0;                 // producer: tiles of A to prefetch into L2 ahead of the shared-memory ring
   // training: Dropout after the activation (modeling.py:121) applied from a keep-bit array (bit i = element i of
   // the [M,N] output, k_train.cu dropout_bits); bf16 outputs, N % 32 == 0
   const uint32_t* drop_bits = nullptr;
@@ -277,10 +275,6 @@ __device__ __forceinline__ void epilogue_rows(const TcEpilogue& ep, const CUtens
         }
       }
       tmem_ld_wait();
-      if (ep.f32_box) {                 // the previous round's box has left the staging tile
-        if (lane == 0) bulk_store_wait_read();
-        __syncwarp();
-      }
 #pragma unroll
       for (int j = 0; j < 4; ++j) st_shared_v4(my_row + ((j ^ sw) << 4), r[4 * j], r[4 * j + 1], r[4 * j + 2], r[4 * j + 3]);
       __syncwarp();
@@ -300,9 +294,10 @@ __device__ __forceinline__ void epilogue_rows(const TcEpilogue& ep, const CUtens
               if (seg > 0) obase = seg == 1 ? ep.out_seg[0] : ep.out_seg[1];
               orow = m - seg * seg_rows;
             }
-            float* o = obase + orow * N + col;
+            // the output address is formed at each store, not once above: at the 96-register cap that leaves ptxas less to spill
             if (atomic) {
               // one 16-byte vector reduction instead of four scalar ones (split-K weight gradients)
+              float* o = obase + orow * N + col;
               asm volatile("red.global.add.v4.f32 [%0], {%1, %2, %3, %4};" ::"l"(o), "f"(v.x), "f"(v.y), "f"(v.z), "f"(v.w)
                            : "memory");
             } else {
@@ -312,21 +307,9 @@ __device__ __forceinline__ void epilogue_rows(const TcEpilogue& ep, const CUtens
               if (ep.act == VIT3D_ACT_GELU) { v.x = gelu_fast(v.x); v.y = gelu_fast(v.y); v.z = gelu_fast(v.z); v.w = gelu_fast(v.w); }
               v.x += res[i].x; v.y += res[i].y; v.z += res[i].z; v.w += res[i].w;
               if (ep.round_tf32) { v.x = round_tf32(v.x); v.y = round_tf32(v.y); v.z = round_tf32(v.z); v.w = round_tf32(v.w); }
-              if (ep.f32_box)     // finished values go back to their staging slot; the [32 x 16] box leaves by one TMA store
-                st_shared_v4(stage + row * 64 + ((chunk ^ ((row >> 1) & 3)) << 4), __float_as_uint(v.x), __float_as_uint(v.y),
-                             __float_as_uint(v.z), __float_as_uint(v.w));
-              else
-                *reinterpret_cast<float4*>(o) = v;
+              *reinterpret_cast<float4*>(obase + orow * N + col) = v;
             }
           }
-        }
-      }
-      if (ep.f32_box) {
-        fence_proxy_async_smem();
-        __syncwarp();
-        if (lane == 0) {
-          tma_store_2d(tmC, stage, n_base + c, m_base);
-          bulk_store_commit();
         }
       }
       __syncwarp();
@@ -464,23 +447,19 @@ __device__ __forceinline__ uint32_t gelu_pair_bf16_h2(__half2 x) {
   return pack2_bf16(f.x, f.y);
 }
 
-// WIDE (CW == 64, no pre-activation output): the warp's whole 32 x 64 slice is staged as ONE panel with
-// 128-byte rows (128B swizzle, 4 KB) and leaves by one bulk tensor store per tile instead of two stores of
-// 64-byte rows - half the TMA row transactions, and the wait for the previous store moves a whole tile away.
 //   MODE bit 3: the training fc1 (needs bits 0-2): output = gelu(v) * keep * scale, and the `pre` output receives
 //               d act / d pre = gelu'(v) * keep * scale (TcEpilogue::store_dact).  `keep` = the CW / 32 words of keep
 //               bits of this thread's row (fetched by the caller before the accumulator wait; 0 for rows >= M, all
 //               ones when the call has no dropout)
-template <int CW, int MODE, bool WIDE = false>
+template <int CW, int MODE>
 __device__ __forceinline__ void epilogue_bf16_lean(const CUtensorMap* tmC, const CUtensorMap* tmPre, uint32_t taddr,
                                                    uint32_t stage, uint32_t bias_f32, uint32_t bias_h2, int lane,
                                                    int m_base, int n_base, const uint32_t* keep = nullptr,
                                                    float drop_scale = 1.f) {
   constexpr bool BIAS = (MODE & 1) != 0, GELU = (MODE & 2) != 0, PRE = (MODE & 4) != 0, DROP = (MODE & 8) != 0;
-  static_assert(!WIDE || (CW == 64 && !PRE), "wide staging: 64 columns per warp, no pre-activation copy");
   static_assert(!DROP || (GELU && PRE), "dropout variant = training fc1 (bias + GELU + pre-activation)");
-  const uint32_t my_row = stage + lane * (WIDE ? 128 : 64);
-  const int sw = WIDE ? (lane & 7) : ((lane >> 1) & 3);
+  const uint32_t my_row = stage + lane * 64;
+  const int sw = (lane >> 1) & 3;
 #pragma unroll
   for (int c = 0; c < CW; c += 32) {
     uint32_t r[32];
@@ -553,21 +532,15 @@ __device__ __forceinline__ void epilogue_bf16_lean(const CUtensorMap* tmC, const
 #pragma unroll
       for (int j = 0; j < 16; ++j) w[j] = GELU ? gelu_pair_bf16(v[2 * j], v[2 * j + 1]) : pack2_bf16(v[2 * j], v[2 * j + 1]);
     }
-    if (!WIDE || c == 0) {
-      if (lane == 0) bulk_store_wait_read();    // the previous store has finished reading the staging tile
-      __syncwarp();
-    }
-    const int j0 = WIDE ? c / 8 : 0;            // 16-byte chunk index of column c within the staged row
+    if (lane == 0) bulk_store_wait_read();      // the previous store has finished reading the staging tile
+    __syncwarp();
 #pragma unroll
-    for (int j = 0; j < 4; ++j)
-      st_shared_v4(my_row + (((j0 + j) ^ sw) << 4), w[4 * j], w[4 * j + 1], w[4 * j + 2], w[4 * j + 3]);
-    if (!WIDE || c + 32 == CW) {
-      fence_proxy_async_smem();
-      __syncwarp();
-      if (lane == 0) {
-        tma_store_2d(tmC, stage, WIDE ? n_base : n_base + c, m_base);
-        bulk_store_commit();
-      }
+    for (int j = 0; j < 4; ++j) st_shared_v4(my_row + ((j ^ sw) << 4), w[4 * j], w[4 * j + 1], w[4 * j + 2], w[4 * j + 3]);
+    fence_proxy_async_smem();
+    __syncwarp();
+    if (lane == 0) {
+      tma_store_2d(tmC, stage, n_base + c, m_base);
+      bulk_store_commit();
     }
   }
 }

@@ -477,7 +477,7 @@ class AttnCoreFn(torch.autograd.Function):
         qkv = _c(qkv.to(ad))
         out = torch.empty(B, S, A, device=qkv.device, dtype=ad)
         probs = None
-        if vis and prec == "bf16" and _STATE.get("probs_padded", True) and _lib.lib().vit3d_attn_padded_supported(S, heads, D):
+        if vis and prec == "bf16" and _lib.lib().vit3d_attn_padded_supported(S, heads, D):
             # rows padded to 72 floats (9 whole 32-byte sectors): sector-aligned stores; callers get the [..., :S] view -
             # the shape and values of the reference's attention_probs (modeling.py:89-90), not contiguous
             ld = 72

@@ -17,7 +17,6 @@ from __future__ import annotations
 
 import copy
 import math
-import os
 
 import torch
 import torch.nn as nn
@@ -93,10 +92,6 @@ class Mlp(nn.Module):
         self._init_weights()
         self.precision = F.get_precision()
         self._site = 1
-        # single-kernel fc1 -> GELU -> fc2 (+ residual, + next LayerNorm) inference path (BF16 mode, hidden 256,
-        # mlp_dim % 256 == 0): the (M, mlp_dim) intermediate never reaches HBM.  VIT3D_FUSED_MLP=0 composes the
-        # two GEMMs instead.
-        self.fused = os.environ.get("VIT3D_FUSED_MLP", "1") == "1"
 
     def _init_weights(self):
         nn.init.xavier_uniform_(self.fc1.weight)
@@ -113,7 +108,7 @@ class Mlp(nn.Module):
             prec = self.precision
             infer = (not (self.training and self.dropout.p > 0.0) and residual is not None
                      and not torch.is_grad_enabled())
-            can_fuse = (infer and self.fused and prec == "bf16" and self.fc1.weight.is_contiguous()
+            can_fuse = (infer and prec == "bf16" and self.fc1.weight.is_contiguous()
                         and self.fc2.weight.is_contiguous()
                         and F.mlp_fused_ln_supported(x.numel() // x.shape[-1], x.shape[-1], self.fc1.weight.shape[0]))
             if final:
@@ -138,7 +133,7 @@ class Mlp(nn.Module):
         if train and step is None:
             step = F.next_dropout_step()
         if (not train and prec == "bf16" and residual is not None and not torch.is_grad_enabled()
-                and self.fused and x.is_cuda and self.fc1.weight.is_contiguous() and self.fc2.weight.is_contiguous()
+                and x.is_cuda and self.fc1.weight.is_contiguous() and self.fc2.weight.is_contiguous()
                 and F.mlp_fused_supported(x.numel() // x.shape[-1], x.shape[-1], self.fc1.weight.shape[0])):
             # inference: one kernel, the (M, mlp_dim) intermediate stays in TMEM / shared memory
             return F.mlp_fused(x, self.fc1.weight, self.fc1.bias, self.fc2.weight, self.fc2.bias, residual)

@@ -52,53 +52,38 @@ const char* vit3d_last_error(void);
 int vit3d_device_info(int* sm_count, int* cc);
 /* number of kernels this library has launched in this process so far */
 unsigned long long vit3d_launch_count(void);
-/* Tuning switches: select between kernel variants at run time (for A/B timing; results agree to rounding).
- *   VIT3D_TUNE_EPI_PANEL     1 (default): fp32-output GEMMs with N % 256 == 0 (out-projection, fc2, fp32 data
- *                            gradients) run the TMA-panel kernel (residual fetched and result stored by bulk
- *                            tensor copies); 0: the generic epilogue.  Env VIT3D_EPI_PANEL.
+/* Tuning switches: test and probe hooks, not user options.  Each selects between kernel variants that agree to
+ * rounding, so that tests can check every variant and probes can time them in one process.  Process-wide; the
+ * defaults below are the variants in use, and only vit3d_set_tuning changes them.  Keys 0, 2, 3, 4, 10 and 13 are
+ * retired: vit3d_set_tuning and vit3d_get_tuning return VIT3D_ERR_INVALID for them (as for any unknown key).
  *   VIT3D_TUNE_ATTN_THREADS  0 (default: chosen per shape), 640 or 512 threads per attention-forward CTA.
- *                            Env VIT3D_ATTN_THREADS.
- *   VIT3D_TUNE_EPI_LEAN      1 (default): compile-time specialised epilogue (bias from shared memory, packed
- *                            half GELU) for bf16-output GEMMs with full column tiles; 0: generic epilogue.
- *                            Env VIT3D_EPI_LEAN.
- *   VIT3D_TUNE_STORE_WIDE    0 (default): 32 x 32 bf16 staging panels, 4-stage A ring; 1: 32 x 64 panels (128-byte
- *                            rows, one bulk tensor store per warp and tile) with a 2-stage ring - measured
- *                            slower (the ring is too shallow).  Env VIT3D_STORE_WIDE.
- *   VIT3D_TUNE_L2_AHEAD      tiles of the A operand the TMA producer prefetches into L2 ahead of its shared-
- *                            memory ring (default 0 = off: measured no gain, the long operand latency under
- *                            write-saturated HBM is not an L2 miss).  Env VIT3D_L2_AHEAD.
  *   VIT3D_TUNE_MLP_PAIR      0 (default): one CTA per 128-row tile of the fused MLP; 1: clusters of two CTAs that
  *                            share every weight k-block by TMA multicast (half the L2 reads; measured equal -
  *                            the kernel is bound by its GELU / final epilogue, not by L2); 2: cta_group::2 pairs; 3: the
  *                            128-column-chunk kernel with double-buffered fc1 accumulator and GELU tile (k_tc_mlp3.cu,
- *                            measured equal).  Env VIT3D_MLP_PAIR.
+ *                            measured equal).
  *   VIT3D_TUNE_WGRAD_RED     1 (default): split-K weight-gradient tiles are added into the gradient buffer by the
  *                            TMA unit (cp.reduce.async.bulk.tensor, fp32 add at the L2); 0: red.global.add.v4.f32
  *                            from the epilogue warps (~1 element per clock and SM); 2: as 1 with 256-row tiles for the large
- *                            products (measured equal).  Env VIT3D_WGRAD_RED.
+ *                            products (measured equal).
  *   VIT3D_TUNE_RES_PAIR      0 (default): independent CTAs; 1: deep-K Linear + residual + LayerNorm products (fc2) run
  *                            on clusters of two CTAs that share every weight k-block by TMA multicast (measured
- *                            equal: not bound by L2 operand delivery).  Env VIT3D_RES_PAIR.
+ *                            equal: not bound by L2 operand delivery).
  *   VIT3D_TUNE_ATTN_TF32     1 (default): TF32-mode attention forward (65 tokens, 256 channels) on mma.sync tf32 in
- *                            (volume, 4-head) units; 0: the generic fp32 SIMT kernel.  Env VIT3D_ATTN_TF32.
- *   VIT3D_TUNE_F32_BOX       0 (default): fp32 GEMM outputs as 64-byte row segments stored by the epilogue warps; 1: dense rows
- *                            leave as [32 x 16] TMA boxes (measured equal in TF32 mode).  Env VIT3D_F32_BOX.
+ *                            (volume, 4-head) units; 0: the generic fp32 SIMT kernel.
  *   VIT3D_TUNE_PATCH_TALL    0 (default): 128-row tiles; 1: the TF32 patch-embedding GEMM of large batches runs 256-row
  *                            tiles (two TMEM accumulators sharing each weight k-block; measured 124 vs 117 us at
- *                            batch 1024).  Env VIT3D_PATCH_TALL.
+ *                            batch 1024).
  *   VIT3D_TUNE_PATCH_CLUSTER 0 (default): independent CTAs; 2 / 4: the patch-embedding GEMM of large batches runs on
  *                            clusters of 2 / 4 CTAs that fetch every filter-bank k-block once (TMA multicast; measured
- *                            equal).  Env VIT3D_PATCH_CLUSTER.
- *   VIT3D_TUNE_PATCH_TF32    1 (default): TF32 mode rounds the volume to nearest TF32 and runs the tensor-core patch
- *                            embedding; 0: exact fp32 gather + SIMT GEMM.  Env VIT3D_PATCH_TF32.
- *   VIT3D_TUNE_ATTN_FWD_UNIT bf16 attention forward: 0 one volume per CTA (bulk-copy staged); 1 (volume, 4-head) units with
- *                            TMA boxes when no probabilities are written; 2 always.  Env VIT3D_ATTN_FWD_UNIT.
+ *                            equal).
+ *   VIT3D_TUNE_ATTN_FWD_UNIT bf16 attention forward: 0 (default) one volume per CTA (bulk-copy staged); 1 (volume, 4-head)
+ *                            units with TMA boxes when no probabilities are written; 2 always.
  *   VIT3D_TUNE_ATTN_BWD      1 (default): attention backward in (volume, 4-head) units, 4-warp CTAs, TMA boxes; 0: one
- *                            16-warp CTA per volume with per-row bulk copies.  Env VIT3D_ATTN_BWD. */
-enum { VIT3D_TUNE_EPI_PANEL = 0, VIT3D_TUNE_ATTN_THREADS = 1, VIT3D_TUNE_EPI_LEAN = 2, VIT3D_TUNE_STORE_WIDE = 3,
-       VIT3D_TUNE_L2_AHEAD = 4, VIT3D_TUNE_MLP_PAIR = 5, VIT3D_TUNE_WGRAD_RED = 6, VIT3D_TUNE_ATTN_BWD = 7,
-       VIT3D_TUNE_RES_PAIR = 8, VIT3D_TUNE_ATTN_TF32 = 9, VIT3D_TUNE_F32_BOX = 10, VIT3D_TUNE_PATCH_TALL = 11,
-       VIT3D_TUNE_PATCH_CLUSTER = 12, VIT3D_TUNE_PATCH_TF32 = 13, VIT3D_TUNE_ATTN_FWD_UNIT = 14, VIT3D_TUNE_COUNT = 15 };
+ *                            16-warp CTA per volume with per-row bulk copies. */
+enum { VIT3D_TUNE_ATTN_THREADS = 1, VIT3D_TUNE_MLP_PAIR = 5, VIT3D_TUNE_WGRAD_RED = 6, VIT3D_TUNE_ATTN_BWD = 7,
+       VIT3D_TUNE_RES_PAIR = 8, VIT3D_TUNE_ATTN_TF32 = 9, VIT3D_TUNE_PATCH_TALL = 11, VIT3D_TUNE_PATCH_CLUSTER = 12,
+       VIT3D_TUNE_ATTN_FWD_UNIT = 14, VIT3D_TUNE_COUNT = 15 };
 int vit3d_set_tuning(int key, int value);
 int vit3d_get_tuning(int key);
 /* bytes per "act" element for a precision mode */

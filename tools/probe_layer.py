@@ -83,41 +83,32 @@ yn = torch.empty(M, H, device=dev, dtype=bf)
 mean = torch.empty(M, device=dev)
 rstd = torch.empty(M, device=dev)
 
-def gemm_suite(tag):
-    report(f"qkv GEMM {tag}", timeit(lambda: linear(xn, w_qkv, wl_qkv, b_qkv, None, qkv, None, 0, 3 * H, H)),
+def gemm_suite():
+    report("qkv GEMM", timeit(lambda: linear(xn, w_qkv, wl_qkv, b_qkv, None, qkv, None, 0, 3 * H, H)),
            2.0 * M * 3 * H * H, M * H * 2 + M * 3 * H * 2)
-    report(f"fc1 GEMM + GELU {tag}", timeit(lambda: linear(xn, w1, wl1, b1, None, h, None, 1, d, H)),
+    report("fc1 GEMM + GELU", timeit(lambda: linear(xn, w1, wl1, b1, None, h, None, 1, d, H)),
            2.0 * M * d * H, M * H * 2 + M * d * 2)
-    report(f"fc1 GEMM + GELU + pre (training) {tag}", timeit(lambda: linear(xn, w1, wl1, b1, None, h, pre, 1, d, H)),
+    report("fc1 GEMM + GELU + pre (training)", timeit(lambda: linear(xn, w1, wl1, b1, None, h, pre, 1, d, H)),
            2.0 * M * d * H, M * H * 2 + 2 * M * d * 2)
-    report(f"fc1 GEMM + bias, no act {tag}", timeit(lambda: linear(xn, w1, wl1, b1, None, h, None, 0, d, H)),
+    report("fc1 GEMM + bias, no act", timeit(lambda: linear(xn, w1, wl1, b1, None, h, None, 0, d, H)),
            2.0 * M * d * H, M * H * 2 + M * d * 2)
-    report(f"out-proj GEMM + residual {tag}", timeit(lambda: linear(ctx, w_o, wl_o, b_o, x32, y32, None, 0, H, H)),
+    report("out-proj GEMM + residual", timeit(lambda: linear(ctx, w_o, wl_o, b_o, x32, y32, None, 0, H, H)),
            2.0 * M * H * H, M * H * 2 + 2 * M * H * 4)
-    report(f"fc2 GEMM + residual {tag}", timeit(lambda: linear(h, w2, wl2, b2, x32, y32, None, 0, H, d)),
+    report("fc2 GEMM + residual", timeit(lambda: linear(h, w2, wl2, b2, x32, y32, None, 0, H, d)),
            2.0 * M * d * H, M * d * 2 + 2 * M * H * 4)
     if L.vit3d_linear_ln_supported(M, H, H):
-        report(f"out-proj GEMM + residual + LN (fused) {tag}",
+        report("out-proj GEMM + residual + LN (fused)",
                timeit(lambda: call("vit3d_linear_ln_fwd", ptr(ctx), ptr(wl_o), ptr(b_o), ptr(x32), ptr(y32), ptr(gamma),
                                    ptr(beta), 1e-6, ptr(yn), None, None, M, H, H, stream())),
                2.0 * M * H * H, M * H * 2 + 2 * M * H * 4 + M * H * 2)
-        report(f"fc2 GEMM + residual + LN (fused) {tag}",
+        report("fc2 GEMM + residual + LN (fused)",
                timeit(lambda: call("vit3d_linear_ln_fwd", ptr(h), ptr(wl2), ptr(b2), ptr(x32), ptr(y32), ptr(gamma),
                                    ptr(beta), 1e-6, ptr(yn), None, None, M, H, d, stream())),
                2.0 * M * d * H, M * d * 2 + 2 * M * H * 4 + M * H * 2)
 
 
-# tuning keys (include/vit3d.h): 0 panel kernel, 1 attention threads, 2 lean epilogue, 3 wide staging, 4 L2 look-ahead,
-# 5 fused-MLP weight multicast
-for ahead in (0,):
-    L.vit3d_set_tuning(4, ahead)
-    gemm_suite(f"[l2_ahead={ahead}]")
-L.vit3d_set_tuning(4, 0)
-L.vit3d_set_tuning(2, 0)
-L.vit3d_set_tuning(0, 0)
-gemm_suite("[generic epilogues]")
-L.vit3d_set_tuning(2, 1)
-L.vit3d_set_tuning(0, 1)
+# tuning keys (include/vit3d.h): 1 attention threads, 5 fused-MLP weight multicast
+gemm_suite()
 w2h = w2.to(torch.float16)
 for pair in (0, 1):
     L.vit3d_set_tuning(5, pair)

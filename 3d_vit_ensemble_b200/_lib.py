@@ -51,6 +51,7 @@ SIGNATURES = {
     "vit3d_patch_embed_ws_bytes": (_sz, [_i] * 9),
     "vit3d_patch_embed_fwd": (_i, [_p, _p, _p, _p, _p, _p, _i, _i, _i, _i, _i, _i, _i, _i, _i, _p, _sz, _p]),
     "vit3d_patch_embed_bwd": (_i, [_p, _p, _p, _p, _p, _p, _i, _i, _i, _i, _i, _i, _i, _i, _i, _p, _sz, _p]),
+    "vit3d_patch_embed_dgrad": (_i, [_p, _p, _p, _p, _i, _i, _i, _i, _i, _i, _i, _i, _i, _p, _sz, _p]),
     "vit3d_ln_fwd": (_i, [_p, _p, _p, _p, _i, _p, _p, _i, _i, _f, _p]),
     "vit3d_ln_bwd": (_i, [_p, _p, _p, _p, _p, _p, _p, _p, _p, _i, _i, _p]),
     "vit3d_linear_fwd": (_i, [_p, _i, _i, _p, _p, _p, _p, _p, _i, _p, _i, _i, _i, _i, _i, _p]),

@@ -200,6 +200,46 @@ int vit3d_patch_embed_bwd(const float* x, const float* dtokens, float* dw, float
   return launch_embed_param_grads(dtokens, dpos, dcls, B, S, H, st);
 }
 
+int vit3d_patch_embed_dgrad(const float* dtokens, const float* w, const void* w_t_lp, float* dx, int B, int X, int Y, int Z,
+                            int p0, int p1, int p2, int H, int prec, void* ws, size_t ws_bytes, vit3d_stream_t stream) {
+  V3_REQUIRE(B >= 0 && p0 > 0 && p1 > 0 && p2 > 0 && X >= p0 && Y >= p1 && Z >= p2 && H > 0, "patch_embed_dgrad: bad shape");
+  if (B == 0) return VIT3D_OK;
+  V3_REQUIRE(dtokens && w && dx, "patch_embed_dgrad: null pointer");
+  V3_REQUIRE(ws && ws_bytes >= vit3d_patch_embed_ws_bytes(B, X, Y, Z, p0, p1, p2, H, prec), "patch_embed_dgrad: workspace too small");
+  cudaStream_t st = as_stream(stream);
+  const int P = (X / p0) * (Y / p1) * (Z / p2), Kp = p0 * p1 * p2, S = P + 1;
+  int rc;
+  const bool aligned = ((reinterpret_cast<uintptr_t>(dtokens) | reinterpret_cast<uintptr_t>(dx) |
+                         reinterpret_cast<uintptr_t>(w_t_lp)) & 15) == 0;
+  if (prec != VIT3D_PREC_FP32 && w_t_lp && aligned && tc_patch_dgrad_supported(B, X, Y, Z, p0, p1, p2, H)) {
+    // BF16 and TF32 modes: one tcgen05 kernel in TF32, stores straight into dx.  BF16 mode reads the fp32 dtokens as they
+    // are (the tensor core truncates them to TF32, as it does the volume in the forward); TF32 mode keeps its rule that
+    // every GEMM operand is round-to-nearest TF32 and rounds dtokens into the workspace first.
+    const float* a = dtokens;
+    if (prec == VIT3D_PREC_TF32) {
+      V3_REQUIRE((size_t)B * S * H * sizeof(float) <= ws_bytes, "patch_embed_dgrad: workspace too small");
+      float* dr = reinterpret_cast<float*>(ws);
+      rc = launch_round_tf32(dtokens, dr, (long long)B * S * H, st);
+      if (rc != VIT3D_OK) return rc;
+      a = dr;
+    }
+    return tc_patch_dgrad(a, reinterpret_cast<const float*>(w_t_lp), dx, B, X, Y, Z, p0, p1, p2, H, st);
+  }
+  // exact fp32: compact the patch rows of dtokens, dpatches[B*P, Kp] = dY[B*P, H] @ w[H, Kp], inverse im2col into dx
+  float* patches = reinterpret_cast<float*>(ws);
+  float* dY = patches + (size_t)B * P * Kp;
+  rc = launch_gather_patch_rows(dtokens, dY, 1, B, P, H, st);
+  if (rc != VIT3D_OK) return rc;
+  SgemmArgs g;
+  g.A = dY; g.sa_m = H; g.sa_k = 1;
+  g.B = w; g.sb_k = Kp; g.sb_n = 1;
+  g.C = patches; g.ldc = Kp;
+  g.M = B * P; g.N = Kp; g.K = H;
+  rc = launch_sgemm(g, st);
+  if (rc != VIT3D_OK) return rc;
+  return launch_patch_scatter(patches, dx, B, X, Y, Z, p0, p1, p2, st);
+}
+
 // ------------------------------------------------------------------------- LayerNorm
 int vit3d_ln_fwd(const float* x, const float* gamma, const float* beta, void* y, int y_bf16, float* mean, float* rstd,
                  int M, int H, float eps, vit3d_stream_t stream) {

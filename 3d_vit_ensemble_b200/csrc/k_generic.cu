@@ -219,6 +219,68 @@ int launch_patch_gather(const float* x, void* out, int out_f32, int B, int X, in
   return VIT3D_OK;
 }
 
+// Inverse permutation (bit-exact): x[b,0,px*p0+i,py*p1+j,pz*p2+z] = patches[(b*P+p)*Kp + (i*p1+j)*p2+z]; EVERY voxel of x
+// is written, 0 where no patch covers it (the X % p0, Y % p1, Z % p2 remainders Conv3d drops).
+__global__ void patch_scatter_kernel(const float* __restrict__ patches, float* __restrict__ x, long long total, int X, int Y,
+                                     int Z, int p0, int p1, int p2, int nx, int ny, int nz) {
+  const long long Kp = (long long)p0 * p1 * p2;
+  const long long P = (long long)nx * ny * nz;
+  for (long long t = blockIdx.x * (long long)blockDim.x + threadIdx.x; t < total; t += (long long)gridDim.x * blockDim.x) {
+    const int zi = (int)(t % Z), yi = (int)((t / Z) % Y), xi = (int)((t / ((long long)Z * Y)) % X);
+    const long long b = t / ((long long)Z * Y * X);
+    float v = 0.f;
+    if (xi < nx * p0 && yi < ny * p1 && zi < nz * p2) {
+      const int px = xi / p0, i = xi - px * p0, py = yi / p1, j = yi - py * p1, pz = zi / p2, z = zi - pz * p2;
+      const long long p = ((long long)px * ny + py) * nz + pz;
+      v = patches[(b * P + p) * Kp + (i * p1 + j) * p2 + z];
+    }
+    x[t] = v;
+  }
+}
+// Fast path (the patch spans all Z slices, so a patch row of p1*Z floats is contiguous in the volume AND in the patch
+// matrix): four voxels per thread, one 16-byte load and one 16-byte store.  Same permutation, bit for bit.
+__global__ void __launch_bounds__(256) patch_scatter_rows_kernel(const float* __restrict__ patches, float* __restrict__ x,
+                                                                 unsigned total4, int X, int Y, int Z, int p0, int p1, int nx,
+                                                                 int ny) {
+  const unsigned inner = (unsigned)(p1 * Z), yz = (unsigned)(Y * Z), Kp = (unsigned)p0 * inner;
+  const unsigned P = (unsigned)(nx * ny);
+  for (unsigned u = blockIdx.x * blockDim.x + threadIdx.x; u < total4; u += gridDim.x * blockDim.x) {
+    const unsigned e = 4u * u;
+    const unsigned bx = e / yz, rem = e - bx * yz;            // bx = b*X + xi, rem = yi*Z + z
+    const unsigned b = bx / (unsigned)X, xi = bx - b * (unsigned)X;
+    const unsigned py = rem / inner, off = rem - py * inner;
+    float4 v = make_float4(0.f, 0.f, 0.f, 0.f);
+    if (xi < (unsigned)(nx * p0) && py < (unsigned)ny) {
+      const unsigned px = xi / (unsigned)p0, i = xi - px * (unsigned)p0;
+      const size_t src = ((size_t)b * P + px * (unsigned)ny + py) * Kp + i * inner + off;
+      v = *reinterpret_cast<const float4*>(patches + src);
+    }
+    reinterpret_cast<float4*>(x)[u] = v;
+  }
+}
+
+int launch_patch_scatter(const float* patches, float* x, int B, int X, int Y, int Z, int p0, int p1, int p2, cudaStream_t st) {
+  const int nx = X / p0, ny = Y / p1, nz = Z / p2;
+  const long long total = (long long)B * X * Y * Z;
+  if (total == 0) return VIT3D_OK;
+  if (nz == 1 && p2 == Z && (p1 * Z) % 4 == 0 && (Y * Z) % 4 == 0 && total < (1ll << 33) &&
+      ((reinterpret_cast<uintptr_t>(x) | reinterpret_cast<uintptr_t>(patches)) & 15) == 0) {
+    const unsigned total4 = (unsigned)(total / 4);
+    unsigned blocks = (total4 + 255) / 256;
+    const unsigned cap = (unsigned)sm_count() * 16;
+    if (blocks > cap) blocks = cap;
+    patch_scatter_rows_kernel<<<blocks, 256, 0, st>>>(patches, x, total4, X, Y, Z, p0, p1, nx, ny);
+    V3_LAUNCH_CHECK();
+    return VIT3D_OK;
+  }
+  long long blocks = (total + 255) / 256;
+  const long long cap = (long long)sm_count() * 16;
+  if (blocks > cap) blocks = cap;
+  patch_scatter_kernel<<<(int)blocks, 256, 0, st>>>(patches, x, total, X, Y, Z, p0, p1, p2, nx, ny, nz);
+  V3_LAUNCH_CHECK();
+  return VIT3D_OK;
+}
+
 // tokens[b,0,:] = cls + pos[0]  (the patch rows are written by the GEMM epilogue)
 __global__ void cls_rows_kernel(const float* __restrict__ cls, const float* __restrict__ pos, float* __restrict__ tokens,
                                 int B, int S, int H) {

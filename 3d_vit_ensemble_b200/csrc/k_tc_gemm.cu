@@ -670,8 +670,8 @@ int tc_linear_fwd(const TcLinear& t, cudaStream_t st) {
 // Conv3d(kernel = stride = patch) as an im2col-by-TMA GEMM in TF32: the fp32 volume is read exactly once,
 // straight into the swizzled A tiles (no gather pass, no conversion pass); bias, position rows and the
 // "skip the cls row" output remap are fused in the epilogue.
-static int make_tmap_nd(CUtensorMap* out, const void* ptr, int rank, const cuuint64_t* dims, const cuuint64_t* strides_bytes,
-                        const cuuint32_t* box) {
+int make_tmap_nd(CUtensorMap* out, const void* ptr, int rank, const cuuint64_t* dims, const cuuint64_t* strides_bytes,
+                 const cuuint32_t* box) {
   EncodeTiledFn enc = get_encode();
   if (!enc) { set_error("cuTensorMapEncodeTiled unavailable"); return VIT3D_ERR_CUDA; }
   cuuint32_t estr[5] = {1, 1, 1, 1, 1};

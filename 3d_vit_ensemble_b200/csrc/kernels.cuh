@@ -24,6 +24,7 @@ int launch_rowdot(const float* x, long long ldx, const float* w, const float* bi
                   cudaStream_t st);
 int launch_patch_gather(const float* x, void* out, int out_f32, int B, int X, int Y, int Z, int p0, int p1, int p2,
                         cudaStream_t st);
+int launch_patch_scatter(const float* patches, float* x, int B, int X, int Y, int Z, int p0, int p1, int p2, cudaStream_t st);
 int launch_cls_rows(const float* cls, const float* pos, float* tokens, int B, int S, int H, cudaStream_t st);
 int launch_embed_param_grads(const float* dtok, float* dpos, float* dcls, int B, int S, int H, cudaStream_t st);
 int launch_gather_patch_rows(const float* dtok, void* out, int out_f32, int B, int P, int H, cudaStream_t st);

@@ -46,6 +46,11 @@ int tc_gemm_wgrad_seg(const void* dy, const void* x, float* dw0, float* dw1, flo
 bool tc_patch_embed_supported(int B, int X, int Y, int Z, int p0, int p1, int p2, int H);
 int tc_patch_embed_fwd(const float* x, const float* w, const float* bias, const float* pos, float* tokens, int B, int X,
                        int Y, int Z, int p0, int p1, int p2, int H, cudaStream_t st);
+// k_tc_patch_dgrad.cu: dx = d tokens / d x on tcgen05 (TF32), straight into the volume by 5-D TMA stores; w_t is the
+// TF32-rounded transposed filter bank [Kp, H]
+bool tc_patch_dgrad_supported(int B, int X, int Y, int Z, int p0, int p1, int p2, int H);
+int tc_patch_dgrad(const float* dtokens, const float* w_t, float* dx, int B, int X, int Y, int Z, int p0, int p1, int p2,
+                   int H, cudaStream_t st);
 
 // k_tc_mlp3.cu: the fused MLP block with 128-column chunks, fc1 accumulator and GELU tile double buffered (same contract
 // as tc_mlp2_fwd)

@@ -47,6 +47,9 @@ struct TcEpilogue {
 // 2-D row-major tensor map (defined in k_tc_gemm.cu, cached per thread)
 int make_tmap_2d(CUtensorMap* out, const void* ptr, int elem_bytes, long long rows, long long cols, long long ld_elems,
                  int box_rows, int box_cols, int swizzle_bytes);
+// rank-N fp32 tensor map with 128-byte swizzle (defined in k_tc_gemm.cu, not cached)
+int make_tmap_nd(CUtensorMap* out, const void* ptr, int rank, const cuuint64_t* dims, const cuuint64_t* strides_bytes,
+                 const cuuint32_t* box);
 
 // ----------------------------------------------------------------------------- epilogue
 // fast GELU (bf16 outputs, and the fp32 outputs of TF32 mode): x * sigmoid(2u), u = x (c0 + c1 x^2 + c2 x^4) fitted to the exact erf

@@ -85,7 +85,8 @@ def invalidate_weight_shadows() -> None:
 
 
 def lp_weight(w: torch.Tensor, prec: str = "bf16") -> torch.Tensor:
-    """bf16 copy (BF16 mode) or TF32-rounded fp32 copy (TF32 mode) of an fp32 weight."""
+    """bf16 copy (BF16 mode) or TF32-rounded fp32 copy (TF32 mode) of an fp32 weight; "bf16_t" / "tf32_t": the same,
+    transposed to [K, N] (K = product of the trailing dimensions)."""
     cacheable = isinstance(w, torch.nn.Parameter)
     if cacheable:
         ent = _LP_CACHE.get((id(w), prec))
@@ -101,6 +102,8 @@ def lp_weight(w: torch.Tensor, prec: str = "bf16") -> torch.Tensor:
     elif prec == "bf16_t":          # transposed bf16 shadow [K,N] of a [N,K] weight: dgrad operand
         out = torch.empty(w.shape[1], w.shape[0], dtype=torch.bfloat16, device=w.device)
         call("vit3d_transpose_f32_to_bf16", ptr(w.detach()), ptr(out), w.shape[0], w.shape[1], stream())
+    elif prec == "tf32_t":          # transposed TF32 shadow [K,N] of an [N,...] weight: patch-embedding dgrad operand
+        out = lp_weight(w, "tf32").reshape(w.shape[0], -1).t().contiguous()
     else:
         out = torch.empty(w.shape, dtype=torch.float32, device=w.device)
         call("vit3d_round_tf32", ptr(w.detach()), ptr(out), w.numel(), stream())
@@ -119,6 +122,7 @@ class PatchEmbedFn(torch.autograd.Function):
     @staticmethod
     def forward(ctx, x, w, bias, cls, pos, prec):
         _need_cuda(x, w, bias, cls, pos)
+        ctx.x_dtype = x.dtype
         x = _c(x.float())
         B, Cc, X, Y, Z = x.shape
         if Cc != 1:
@@ -149,25 +153,38 @@ class PatchEmbedFn(torch.autograd.Function):
         B, _, X, Y, Z = x.shape
         H, _, p0, p1, p2 = wshape
         dev = x.device
-        targets = [_grad_target(p) for p in ctx.params]
-        direct = all(t is not None for t in targets)
-        if direct:
-            dw, db, dcls, dpos = targets
-        else:
-            dw = torch.zeros(wshape, device=dev)
-            db = torch.zeros(H, device=dev)
-            dcls = torch.zeros(cshape, device=dev)
-            dpos = torch.zeros(pshape, device=dev)
         pid = PREC[prec]
         wsb = _lib.lib().vit3d_patch_embed_ws_bytes(B, X, Y, Z, p0, p1, p2, H, pid)
         ws = torch.empty(wsb, device=dev, dtype=torch.uint8)
-        call("vit3d_patch_embed_bwd", ptr(x), ptr(_c(dtok.float())), ptr(dw), ptr(db), ptr(dcls), ptr(dpos),
-             B, X, Y, Z, p0, p1, p2, H, pid, ptr(ws), wsb, stream())
-        if direct:
-            for p in ctx.params:
-                _grad_done(p)
-            return None, None, None, None, None, None
-        return None, dw, db, dcls, dpos, None
+        dtok = _c(dtok.float())
+        grads = [None] * 6
+        if any(ctx.needs_input_grad[1:5]):
+            targets = [_grad_target(p) for p in ctx.params]
+            direct = all(t is not None for t in targets)
+            if direct:
+                dw, db, dcls, dpos = targets
+            else:
+                dw = torch.zeros(wshape, device=dev)
+                db = torch.zeros(H, device=dev)
+                dcls = torch.zeros(cshape, device=dev)
+                dpos = torch.zeros(pshape, device=dev)
+            call("vit3d_patch_embed_bwd", ptr(x), ptr(dtok), ptr(dw), ptr(db), ptr(dcls), ptr(dpos),
+                 B, X, Y, Z, p0, p1, p2, H, pid, ptr(ws), wsb, stream())
+            if direct:
+                for p in ctx.params:
+                    _grad_done(p)
+            else:
+                grads[1:5] = dw, db, dcls, dpos
+        if ctx.needs_input_grad[0]:
+            # d tokens / d x (Conv3d data gradient): BF16 and TF32 modes hand the tensor-core kernel the transposed
+            # TF32-rounded filter bank, fp32 mode takes the exact path from the master weight
+            w = ctx.params[0]
+            w_t = lp_weight(w, "tf32_t") if (prec in ("bf16", "tf32") and w.is_contiguous()) else None
+            dx = torch.empty(x.shape, device=dev, dtype=torch.float32)
+            call("vit3d_patch_embed_dgrad", ptr(dtok), ptr(_c(w.detach())), ptr(w_t), ptr(dx), B, X, Y, Z, p0, p1, p2, H,
+                 pid, ptr(ws), wsb, stream())
+            grads[0] = dx.to(ctx.x_dtype)
+        return tuple(grads)
 
 
 def u8_volumes_to_f32(x_u8: torch.Tensor, mean: float) -> torch.Tensor:

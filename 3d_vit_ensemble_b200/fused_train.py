@@ -498,6 +498,11 @@ def backward_steps(model, saved, dloss: Optional[torch.Tensor] = None, cuts=()):
     ws = torch.empty(wsb, device=dev, dtype=torch.uint8)
     call("vit3d_patch_embed_bwd", ptr(x), ptr(g), G(w), G(emb.patch_embeddings.bias), G(emb.cls_token),
          G(emb.position_embeddings), B, X, Y, Z, p0, p1, p2, H, _BF16, ptr(ws), wsb, st)
+    if saved.get("need_dx"):       # the input volume's gradient (autograd callers whose x requires grad)
+        dx = torch.empty(x.shape, device=dev, dtype=f32)
+        call("vit3d_patch_embed_dgrad", ptr(g), ptr(w), ptr(F.lp_weight(w, "tf32_t")), ptr(dx), B, X, Y, Z, p0, p1, p2, H,
+             _BF16, ptr(ws), wsb, st)
+        saved["dx"] = dx
     for p_ in emb.parameters():
         F._grad_done(p_)
     return G.result(params)
@@ -509,15 +514,18 @@ class VitTrainFn(torch.autograd.Function):
     @staticmethod
     def forward(ctx, model, x, labels, pos_weight, *params):
         loss, saved = forward(model, x, labels, pos_weight)
+        saved["need_dx"] = ctx.needs_input_grad[1]
         ctx.model = model
         ctx.saved = saved
+        ctx.x_dtype = x.dtype
         return loss
 
     @staticmethod
     def backward(ctx, dloss):
         grads = backward(ctx.model, ctx.saved, dloss)
+        dx = ctx.saved.get("dx")
         ctx.saved = None
-        return (None, None, None, None) + tuple(grads)
+        return (None, None if dx is None else dx.to(ctx.x_dtype), None, None) + tuple(grads)
 
 
 def loss(model, x, labels, pos_weight):

@@ -108,6 +108,15 @@ int vit3d_patch_embed_fwd(const float* x, const float* w, const float* bias, con
 int vit3d_patch_embed_bwd(const float* x, const float* dtokens, float* dw, float* dbias, float* dcls, float* dpos,
                           int B, int X, int Y, int Z, int p0, int p1, int p2, int H, int prec,
                           void* ws, size_t ws_bytes, vit3d_stream_t stream);
+/* dx[B,1,X,Y,Z] = d tokens / d x  (written, not accumulated; uncovered voxels get 0).
+ * w_t_lp: the filter bank TRANSPOSED, [Kp, H]: TF32-rounded fp32 (BF16 / TF32 modes) or NULL (FP32 mode, uses w).
+ * ws as for vit3d_patch_embed_fwd (vit3d_patch_embed_ws_bytes).
+ * BF16 / TF32 modes with w_t_lp, 16-byte aligned buffers, H <= 256 and a geometry the tensor-core forward serves: one
+ * tcgen05 kernel (TF32 mode rounds dtokens to nearest TF32 first: two launches).  Otherwise exact fp32: patch-row
+ * compaction, FMA GEMM, inverse im2col (three launches). */
+int vit3d_patch_embed_dgrad(const float* dtokens, const float* w, const void* w_t_lp, float* dx,
+                            int B, int X, int Y, int Z, int p0, int p1, int p2, int H, int prec,
+                            void* ws, size_t ws_bytes, vit3d_stream_t stream);
 
 /* ---------------------------------------------------------------- a4/a5: LayerNorm(eps, biased var, affine)
  * nn.LayerNorm(H, eps=1e-6) at modeling.py:182-183,189,194,242,253.

@@ -67,6 +67,8 @@ SIGNATURES = {
     "vit3d_attn_bwd": (_i, [_p, _p, _p, _i, _i, _i, _i, _i, _p]),
     "vit3d_attn_fwd_padded": (_i, [_p, _p, _p, _i, _i, _i, _i, _i, _p]),
     "vit3d_attn_padded_supported": (_i, [_i, _i, _i]),
+    "vit3d_qkv_attn_fwd": (_i, [_p, _p, _p, _p, _p, _i, _i, _i, _i, _i, _p]),
+    "vit3d_qkv_attn_supported": (_i, [_i, _i, _i]),
     "vit3d_gelu_fwd": (_i, [_p, _p, _ll, _i, _p]),
     "vit3d_gelu_bwd": (_i, [_p, _p, _p, _ll, _i, _p]),
     "vit3d_gelu_dropout_bwd": (_i, [_p, _p, _p, _ll, _i, _f, _ull, _u, _u, _p, _p]),

@@ -397,6 +397,14 @@ int vit3d_attn_fwd_padded(const void* qkv, void* ctx, float* probs, int probs_ld
   return tc_attn_fwd(qkv, ctx, probs, probs_ld, B, S, heads, D, as_stream(stream));
 }
 int vit3d_attn_padded_supported(int S, int heads, int D) { return tc_attn_supported(S, heads, D) ? 1 : 0; }
+int vit3d_qkv_attn_fwd(const void* yn, const void* w_qkv, const float* b_qkv, void* ctx, float* probs, int probs_ld, int B,
+                       int S, int heads, int D, vit3d_stream_t stream) {
+  V3_REQUIRE(yn && w_qkv && b_qkv && ctx, "qkv_attn_fwd: null pointer");
+  V3_REQUIRE(B >= 0 && S > 0 && heads > 0 && D > 0, "qkv_attn_fwd: bad shape");
+  if (!tc_qkv_attn_supported(S, heads, D)) V3_UNSUPPORTED("qkv_attn_fwd: unsupported shape S=%d heads=%d D=%d", S, heads, D);
+  return tc_qkv_attn_fwd(yn, w_qkv, b_qkv, ctx, probs, probs_ld, B, S, heads, D, as_stream(stream));
+}
+int vit3d_qkv_attn_supported(int S, int heads, int D) { return tc_qkv_attn_supported(S, heads, D) ? 1 : 0; }
 int vit3d_attn_bwd(const void* dctx, const void* qkv, void* dqkv, int B, int S, int heads, int D, int prec,
                    vit3d_stream_t stream) {
   V3_REQUIRE(dctx && qkv && dqkv, "attn_bwd: null pointer");

@@ -75,6 +75,11 @@ int tc_attn_fwd(const void* qkv, void* ctx, float* probs, int probs_ld, int B, i
 // TF32 mode: fp32 q | k | v and context, mma.sync tf32 (k_tc_attn.cu); round_out: context rounded to tf32
 int tc_attn_fwd_tf32(const float* qkv, float* ctx, float* probs, int probs_ld, int B, int S, int heads, int D, int round_out,
                      cudaStream_t st);
+// k_tc_qkv_attn.cu: BF16 inference, yn [B*S, 256] bf16 -> q|k|v (w_qkv [768, 256] bf16, b_qkv [768]) -> attention, in
+// one kernel; probs null or rows of 72 floats in a 32-byte aligned buffer
+bool tc_qkv_attn_supported(int S, int heads, int D);
+int tc_qkv_attn_fwd(const void* yn, const void* w_qkv, const float* b_qkv, void* ctx, float* probs, int probs_ld, int B,
+                    int S, int heads, int D, cudaStream_t st);
 // db_q / db_k / db_v (each [heads*D] fp32, all or none): += column sums of dq / dk / dv (the q, k, v bias gradients)
 int tc_attn_bwd(const void* dctx, const void* qkv, void* dqkv, float* db_q, float* db_k, float* db_v, int B, int S,
                 int heads, int D, cudaStream_t st);

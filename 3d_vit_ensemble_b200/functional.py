@@ -480,6 +480,25 @@ def linear_packed(x, w, b, w_lp, prec):
     return y.reshape(*lead, N)
 
 
+def qkv_attn_supported(x, heads: int) -> bool:
+    """Whether qkv_attn runs x [B, S, H] with this head count."""
+    B, S, H = x.shape
+    return H == 256 and x.dtype == torch.bfloat16 and bool(_lib.lib().vit3d_qkv_attn_supported(S, heads, H // heads))
+
+
+def qkv_attn(x, w_lp, b, heads: int, vis: bool):
+    """Inference in BF16 mode: the packed q|k|v projection of x (bf16 weight shadow w_lp, fp32 bias b) and the attention
+    core in one kernel; returns (ctx, probs or None) like linear_packed followed by AttnCoreFn.apply, equal bit for bit."""
+    _need_cuda(x, w_lp, b)
+    B, S, H = x.shape
+    A = w_lp.shape[0] // 3
+    x = _c(x)
+    out = torch.empty(B, S, A, device=x.device, dtype=torch.bfloat16)
+    store = torch.empty(B, heads, S, 72, device=x.device) if vis else None
+    call("vit3d_qkv_attn_fwd", ptr(x), ptr(w_lp), ptr(b), ptr(out), ptr(store), 72, B, S, heads, A // heads, stream())
+    return out, (store[..., :S] if vis else None)
+
+
 # ----------------------------------------------------------------------------- attention core
 class AttnCoreFn(torch.autograd.Function):
     """softmax(q k^T / sqrt(D)) v per (volume, head) (modeling.py:83-96) on the packed qkv matrix."""

@@ -64,9 +64,14 @@ class Attention(nn.Module):
             w = torch.cat((self.query.weight, self.key.weight, self.value.weight), dim=0)
             b = torch.cat((self.query.bias, self.key.bias, self.value.bias), dim=0)
             qkv = F.linear(hidden_states, w, b, prec=prec)
+            ctx, weights = F.AttnCoreFn.apply(qkv, self.num_attention_heads, bool(self.vis), prec)
+        elif prec == "bf16" and F.qkv_attn_supported(hidden_states, self.num_attention_heads):
+            # one kernel: the q|k|v matrix stays on chip
+            _, b, w_lp = F.packed_qkv(self, prec)
+            ctx, weights = F.qkv_attn(hidden_states, w_lp, b, self.num_attention_heads, bool(self.vis))
         else:
             qkv = F.linear_packed(hidden_states, *F.packed_qkv(self, prec), prec)
-        ctx, weights = F.AttnCoreFn.apply(qkv, self.num_attention_heads, bool(self.vis), prec)
+            ctx, weights = F.AttnCoreFn.apply(qkv, self.num_attention_heads, bool(self.vis), prec)
         p = self.attn_dropout.p
         if p > 0.0 and self.training:
             raise Vit3dError("attention_dropout_rate > 0 is not implemented (the reference config fixes it at 0.0, "

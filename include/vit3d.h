@@ -198,6 +198,15 @@ int vit3d_attn_fwd(const void* qkv, void* ctx, float* probs, int B, int S, int h
 int vit3d_attn_fwd_padded(const void* qkv, void* ctx, float* probs, int probs_ld, int B, int S, int heads, int D,
                           vit3d_stream_t stream);
 int vit3d_attn_padded_supported(int S, int heads, int D);
+/* BF16 inference: the q|k|v projection and the attention core in one kernel (S = 65, H = 256, D = 16 or 32; see
+ * vit3d_qkv_attn_supported).  yn [B*S, H] bf16,
+ * w_qkv [3*k*D, H] bf16 (q | k | v row blocks), b_qkv [3*k*D] fp32; ctx [B*S, k*D] bf16; probs null (vis=False) or
+ * [B,k,S,probs_ld] fp32 with probs_ld = 72 and a 32-byte aligned base, padding written as zeros (as
+ * vit3d_attn_fwd_padded).  ctx and probs equal those of vit3d_linear_fwd (bias, bf16 output) followed by
+ * vit3d_attn_fwd / vit3d_attn_fwd_padded bit for bit; the q|k|v matrix is never written. */
+int vit3d_qkv_attn_fwd(const void* yn, const void* w_qkv, const float* b_qkv, void* ctx, float* probs, int probs_ld, int B,
+                       int S, int heads, int D, vit3d_stream_t stream);
+int vit3d_qkv_attn_supported(int S, int heads, int D);
 /* dqkv from dctx (probabilities are recomputed from qkv) */
 int vit3d_attn_bwd(const void* dctx, const void* qkv, void* dqkv, int B, int S, int heads, int D, int prec,
                    vit3d_stream_t stream);

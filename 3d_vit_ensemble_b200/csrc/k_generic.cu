@@ -467,7 +467,11 @@ int launch_ln_bwd(const float* dy, const float* x, const float* mean, const floa
   int rpb = ceil_div(M, 2 * sm_count());
   if (rpb < 8) rpb = 8;
   const int blocks = ceil_div(M, rpb);
-  ln_bwd_kernel<<<blocks, 256, 2 * H * sizeof(float), st>>>(dy, x, mean, rstd, gamma, dres, dx, dgamma, dbeta, M, H, rpb);
+  // [2][H] fp32 column partials: H > 6144 needs more than the default 48 KB (H = 8192, the widest vit3d_ln_bwd accepts: 64 KB)
+  const size_t smem = 2 * (size_t)H * sizeof(float);
+  if (smem > 48 * 1024)
+    V3_CUDA(cudaFuncSetAttribute(ln_bwd_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 2 * 8192 * (int)sizeof(float)));
+  ln_bwd_kernel<<<blocks, 256, smem, st>>>(dy, x, mean, rstd, gamma, dres, dx, dgamma, dbeta, M, H, rpb);
   V3_LAUNCH_CHECK();
   return VIT3D_OK;
 }
